@@ -37,6 +37,7 @@ MODULI = [0x7fffffd8001, 0x7fffffc8001, 0xfffffffc001, 0xffffff6c001, 0xfffffebc
 PLAIN = 1032193
 BATCH = 1024
 NTT_POLYS = 4096  # BASELINE config 2
+DUMP_ITEMS = 64  # ciphertexts of the last timed step written by --dump-outputs: 64 x 2 x 4 x 8192 float64 = 32 MiB
 
 
 def peaks():
@@ -285,6 +286,9 @@ class PluginLegs:
         src = os.path.join(ROOT, "tools", "plugin_probe.cpp")
         try:
             if not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(src):
+                # the tree may be read-only: a missing or stale harness is compiled into a temporary directory
+                import tempfile
+                so = os.path.join(tempfile.mkdtemp(prefix="b200_bench_"), "libplugin_probe.so")
                 subprocess.run(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-pthread", "-o", so, src], check=True)
             C = self.C
             lib = C.CDLL(so)
@@ -339,6 +343,18 @@ class PluginLegs:
         return ok
 
 
+def dump_outputs(directory, out, batch):
+    """The words of a fixed, seeded sample of the batch's results as float64 (exact: every residue is below 2^53), with
+    the batch indices they came from, so that two builds can be compared on identical inputs."""
+    import numpy as np
+    import torch
+    items = np.sort(np.random.default_rng(0).choice(batch, size=min(DUMP_ITEMS, batch), replace=False))
+    words = out[torch.from_numpy(items).to(out.device)].cpu().numpy()
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "mul_relin_out.npy"), words.astype(np.float64))
+    np.save(os.path.join(directory, "mul_relin_out_items.npy"), items.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -348,7 +364,11 @@ def main():
     ap.add_argument("--batch", type=int, default=BATCH)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--quick", action="store_true", help="device-resident loop + rooflines only (for runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help=f"write a fixed sample of {DUMP_ITEMS} multiply+relinearize results of the last timed step to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -419,6 +439,8 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     launches = ctx.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, B)
     if dist is not None:
         tms = torch.tensor([ms], device=dev, dtype=torch.float64)
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)

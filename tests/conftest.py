@@ -43,3 +43,13 @@ def ref():
     if not refseal.have_ref():
         pytest.skip("reference library oracle/_ref/libsealc_ref.so not available")
     return refseal.RefLib.get()
+
+
+@pytest.fixture(scope="session")
+def ref_or_none(request):
+    """The reference library when it is available, else None: the parity checks then compare with the records of its
+    outputs in tests/golden/reference_parity.json."""
+    try:
+        return request.getfixturevalue("ref")
+    except pytest.skip.Exception:
+        return None

@@ -9,7 +9,7 @@ from params import PARAMS
 
 
 @pytest.fixture(scope="module", params=["n4096", "n8192", "n8192_54", "n8192_49"])
-def pair(request, emu_lib, ref):
+def pair(request, emu_lib, ref_or_none):
     n, moduli, t = PARAMS[request.param]
     return pc.Pair(EmuBackend(emu_lib), n, moduli, t)
 
@@ -27,8 +27,8 @@ def test_elementwise(pair):
 
 
 def test_multiply_and_relinearize(pair):
-    m3, rm = pc.check_multiply(pair)
-    pc.check_relin(pair, m3, rm)
+    m3 = pc.check_multiply(pair)
+    pc.check_relin(pair, m3)
 
 
 def test_galois(pair):
@@ -81,14 +81,14 @@ def test_encrypted_roundtrip(pair):
     pc.check_encrypted_roundtrip(pair)
 
 
-def test_n32768_two_level_transform(emu_lib, ref):
+def test_n32768_two_level_transform(emu_lib, ref_or_none):
     """BASELINE config 5 parameters (n=32768, 15 data residues + special): the two-level NTT and K=15 kernels."""
     n, moduli, t = PARAMS["n32768"]
     P = pc.Pair(EmuBackend(emu_lib), n, moduli, t)
     pc.check_context(P)
     pc.check_ntt(P, items=1)
-    m3, rm = pc.check_multiply(P, with_sizes=False)
-    pc.check_relin(P, m3, rm)
+    m3 = pc.check_multiply(P, with_sizes=False)
+    pc.check_relin(P, m3)
     pc.check_galois(P)
     pc.check_plain(P)
     pc.check_modswitch(P)

@@ -16,7 +16,7 @@ def be():
 
 
 @pytest.fixture(scope="module", params=["n4096", "n8192", "n8192_54", "n8192_49", "n16384", "n32768"])
-def pair(request, be, ref):
+def pair(request, be, ref_or_none):
     n, moduli, t = PARAMS[request.param]
     return pc.Pair(be, n, moduli, t)
 
@@ -40,8 +40,8 @@ def test_elementwise(pair):
 
 
 def test_multiply_and_relinearize(pair):
-    m3, rm = pc.check_multiply(pair, with_sizes=pair.n <= 16384)
-    pc.check_relin(pair, m3, rm)
+    m3 = pc.check_multiply(pair, with_sizes=pair.n <= 16384)
+    pc.check_relin(pair, m3)
 
 
 def test_galois(pair):
@@ -96,7 +96,7 @@ def _threads():
 
 
 @pytest.mark.parametrize("name,level", [("n8192", None), ("n8192_54", 0)])
-def test_config2_all_16384_transforms_vs_reference(be, ref, name, level):
+def test_config2_all_16384_transforms_vs_reference(be, ref_or_none, name, level):
     """BASELINE config 2 at FULL size: every one of the 4096 x 4 forward transforms equals the reference's
     ntt_negacyclic_harvey (S/util/ntt.cpp:393-436) word for word (inputs: the fixed-seed splitmix64(0xB200) % q_i generator of
     SURVEY.md App. B); then the inverse returns the input.  Both prime sets of SURVEY.md 8(d): the four default data primes
@@ -116,10 +116,11 @@ def test_config2_all_16384_transforms_vs_reference(be, ref, name, level):
     d = be.to_dev(x)
     ctx.ntt_forward(d, items, level=level)
     got = be.to_host(d)
-    R = refseal.RefLib.get()
+    R = refseal.RefLib.get() if ref_or_none is not None else None
     for i in range(k):
-        exp = R.ntt_forward_mt(int(moduli[i]), x[:, i, :], _threads())
-        pc.eq(got[:, i, :], exp, f"all {items} forward transforms, prime {i}")
+        label = f"all {items} forward transforms, prime {i}"
+        exp = pc.expect(f"{name}/{label}", lambda R: R.ntt_forward_mt(int(moduli[i]), x[:, i, :], _threads()), R)
+        pc.eq(got[:, i, :], exp, label)
     ctx.ntt_inverse(d, items, level=level)
     pc.eq(be.to_host(d), x, "inverse of all transforms")
 

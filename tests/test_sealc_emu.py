@@ -17,12 +17,12 @@ def test_simple_multiply_ffi_sequence(S, ref):
 
 
 @pytest.mark.parametrize("name", ["n4096", "n8192"])
-def test_evaluator_surface(S, ref, name):
+def test_evaluator_surface(S, ref_or_none, name):
     sc.evaluator_surface(S, *PARAMS[name])
 
 
-def test_error_codes(S, ref):
-    sc.error_codes(S, ref, *PARAMS["n4096"])
+def test_error_codes(S, ref_or_none):
+    sc.error_codes(S, ref_or_none, *PARAMS["n4096"])
 
 
 @pytest.mark.parametrize("name", ["n4096", "n8192"])
@@ -40,7 +40,7 @@ def test_chi_sq_dag_small(S, ref):
 
 
 @pytest.mark.parametrize("name", ["n8192"])
-def test_batch_encoder(S, ref, name):
+def test_batch_encoder(S, ref_or_none, name):
     sc.batch_encoder_parity(S, *PARAMS[name])
 
 
@@ -82,7 +82,7 @@ def test_misuse_hresults(S, ref, name):
     sc.misuse_hresults(S, *PARAMS[name])
 
 
-def test_context_validation_sweep(S, ref):
+def test_context_validation_sweep(S, ref_or_none):
     sc.context_validation_sweep(S)
 
 
@@ -95,7 +95,7 @@ def test_combined_calls_isolation(S, ref):
     sc.combined_calls_isolation(S, *PARAMS["n4096"])
 
 
-def test_handle_lifetime_order(S, ref):
+def test_handle_lifetime_order(S, ref_or_none):
     sc.handle_lifetime_order(S, *PARAMS["n4096"])
 
 

@@ -24,12 +24,12 @@ def test_simple_multiply_ffi_sequence(S, ref):
 
 
 @pytest.mark.parametrize("name", ["n4096", "n8192", "n16384"])
-def test_evaluator_surface(S, ref, name):
+def test_evaluator_surface(S, ref_or_none, name):
     sc.evaluator_surface(S, *PARAMS[name])
 
 
-def test_error_codes(S, ref):
-    sc.error_codes(S, ref, *PARAMS["n4096"])
+def test_error_codes(S, ref_or_none):
+    sc.error_codes(S, ref_or_none, *PARAMS["n4096"])
 
 
 def test_batched_multiply_relin_seam(S, ref):
@@ -107,13 +107,13 @@ def test_config4_chi_sq_dag_n16384(S, ref):
     sc.chi_sq_dag(S, *PARAMS["n16384"], evaluations=3)
 
 
-def test_config5_rotate_multiply_plain_sweep_n32768(S, ref):
+def test_config5_rotate_multiply_plain_sweep_n32768(S, ref_or_none):
     """BASELINE config 5 (n=32768, 15 data residues): rotate_rows + multiply_plain sweep."""
     sc.rotate_multiply_plain_sweep(S, *PARAMS["n32768"], steps=(1, 2, 4, 64, 1024, 8192))
 
 
 @pytest.mark.parametrize("name", ["n8192", "n16384", "n32768"])
-def test_batch_encoder(S, ref, name):
+def test_batch_encoder(S, ref_or_none, name):
     sc.batch_encoder_parity(S, *PARAMS[name])
 
 
@@ -155,7 +155,7 @@ def test_misuse_hresults(S, ref, name):
     sc.misuse_hresults(S, *PARAMS[name])
 
 
-def test_context_validation_sweep(S, ref):
+def test_context_validation_sweep(S, ref_or_none):
     sc.context_validation_sweep(S)
 
 
@@ -167,7 +167,7 @@ def test_combined_calls_isolation(S, ref):
     sc.combined_calls_isolation(S, *PARAMS["n4096"])
 
 
-def test_handle_lifetime_order(S, ref):
+def test_handle_lifetime_order(S, ref_or_none):
     sc.handle_lifetime_order(S, *PARAMS["n4096"])
 
 
